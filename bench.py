@@ -1,7 +1,7 @@
 # coding=utf-8
 """Benchmark of the Multiverse ConvRNN hot path on B200 (contract: see the task statement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c3] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c4|c3|c5] [--impl reference] [--dump-outputs DIR]
   (N>1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 A "step" is one pass of the hot path over one batch of synthetic trajectories
@@ -28,6 +28,8 @@ import time
 import numpy as np
 import torch
 
+# the benchmark runs from a built tree that may be read-only: compile no bytecode into it
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 
@@ -162,6 +164,27 @@ def run_reference(args, wl):
   print(json.dumps(line), flush=True)
 
 
+DUMP_MAX_ELEMENTS = 2 << 20      # per array: 8 MB in float32; the five largest outputs stay under 64 MB together
+
+
+def dump_outputs(out_dir, arrays):
+  """Writes each named output as out_dir/<name>.npy: float32 stays float32, everything else (ids included) becomes
+  float64.  An array of more than DUMP_MAX_ELEMENTS elements is replaced by a sample of its flattened elements at
+  sorted random positions drawn from a generator seeded with the name and the size, so two runs of the same
+  arguments store the same positions."""
+  import zlib
+  os.makedirs(out_dir, exist_ok=True)
+  for name, t in arrays.items():
+    flat = t.detach().reshape(-1) if torch.is_tensor(t) else torch.from_numpy(np.ascontiguousarray(t)).reshape(-1)
+    n = flat.numel()
+    if n > DUMP_MAX_ELEMENTS:
+      rng = np.random.default_rng(zlib.crc32(("%s/%d" % (name, n)).encode()))
+      idx = np.unique(rng.integers(0, n, size=DUMP_MAX_ELEMENTS))
+      flat = flat[torch.from_numpy(idx).to(flat.device)]
+    a = flat.cpu().numpy()
+    np.save(os.path.join(out_dir, name + ".npy"), a if a.dtype == np.float32 else a.astype(np.float64))
+
+
 def setup():
   """Device + (for N > 1) the NCCL process group of this rank: (world, rank, local, dev, dist or None)."""
   from multiverse_b200 import build
@@ -211,8 +234,9 @@ def ddp_equivalence(ctx):
   return res
 
 
-def run_train(args, name, ctx, steps, warmup, cpu_baseline=True):
-  """Workload c5: one Trainer.step (code/pred_models.py:1719-1742) per timed step.  Returns the record on rank 0."""
+def run_train(args, name, ctx, steps, warmup, cpu_baseline=True, dump_dir=None):
+  """Workload c5: one Trainer.step (code/pred_models.py:1719-1742) per timed step.  Returns the record on rank 0;
+  with dump_dir, rank 0 writes the losses of the last timed step there (dump_outputs)."""
   from multiverse_b200 import ops, synthetic
   from multiverse_b200.train_engine import TrainEngine
   wl = WORKLOADS[name]
@@ -281,10 +305,15 @@ def run_train(args, name, ctx, steps, warmup, cpu_baseline=True):
     sampler.start()
   ops.reset_launch_count()
   eng.allreduce_events = []
-  ms_total = timed(lambda: eng.train_step(feeds, lr, dist, mb), steps)
+  last = {}
+  step_fn = lambda: eng.train_step(feeds, lr, dist, mb)
+  ms_total = timed((lambda: last.__setitem__("out", step_fn())) if dump_dir else step_fn, steps)
   launches = ops.launch_count()
   ar_events, eng.allreduce_events = eng.allreduce_events, None
   clocks = sampler.stop() if rank == 0 else None
+  if dump_dir and rank == 0:
+    losses, wd = last.pop("out")
+    dump_outputs(dump_dir, dict(losses=losses, wd_loss=torch.as_tensor(wd).reshape(1)))
   ar = None
   if ar_events:
     # the one collective of the path (85 MB fp32 gradient bucket), device time per step.  A rank that arrives early
@@ -362,6 +391,8 @@ def main():
   ap.add_argument("--planes", type=int, default=2)
   ap.add_argument("--no-cpu-baseline", action="store_true")
   ap.add_argument("--no-extras", action="store_true", help="default run: skip the c3 / c5 sub-records")
+  ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                  help="write what the measured workload's last timed step returned as DIR/<name>.npy")
   args = ap.parse_args()
   extras = args.workload is None and not args.no_extras and not args.global_batch
   args.workload = args.workload or "c4"
@@ -372,12 +403,12 @@ def main():
   ctx = setup()
   world, rank, local, dev, dist = ctx
   run = run_train if wl.get("train") else run_infer
-  line = run(args, args.workload, ctx, args.steps, args.warmup)
+  line = run(args, args.workload, ctx, args.steps, args.warmup, dump_dir=args.dump_outputs)
   if extras:
     # the other two north_star workloads in the same invocation, at the same N and in the same process group
     sub = {}
-    sub["c3"] = run_infer(args, "c3", ctx, max(args.steps, 10), args.warmup, cpu_baseline=False)
-    sub["c5"] = run_train(args, "c5", ctx, max(2, min(args.steps, 3)), args.warmup, cpu_baseline=False)
+    sub["c3"] = run_infer(args, "c3", ctx, args.steps, args.warmup, cpu_baseline=False)
+    sub["c5"] = run_train(args, "c5", ctx, args.steps, args.warmup, cpu_baseline=False)
     chk = ddp_equivalence(ctx) if world > 1 else None
     if rank == 0:
       sub["c5"]["ddp_equivalence"] = chk if chk is not None else "n/a at N=1 (tests/test_ddp_gpu.py runs it on 2 GPUs)"
@@ -388,8 +419,9 @@ def main():
     dist.destroy_process_group()
 
 
-def run_infer(args, name, ctx, steps, warmup, cpu_baseline=True):
-  """Workloads c4 / c3: one forward (all decoders) per timed step.  Returns the record on rank 0."""
+def run_infer(args, name, ctx, steps, warmup, cpu_baseline=True, dump_dir=None):
+  """Workloads c4 / c3: one forward (all decoders) per timed step.  Returns the record on rank 0; with dump_dir,
+  rank 0 writes the forward outputs of the last timed step there (dump_outputs)."""
   from multiverse_b200 import ops, synthetic
   from multiverse_b200.engine import ConvRNNEngine
   wl = WORKLOADS[name]
@@ -489,8 +521,19 @@ def run_infer(args, name, ctx, steps, warmup, cpu_baseline=True):
   ops.reset_launch_count()
   if not use_graph:
     eng.cell_events = []
-  ms_total = timed(step_fn, steps)
+  last = {}
+  ms_total = timed((lambda: last.__setitem__("out", step_fn())) if dump_dir else step_fn, steps)
   launches = ops.launch_count()
+  if dump_dir and rank == 0:
+    # before the untimed launch-by-launch region below: graph replays return their static output buffers
+    out = last.pop("out")
+    res = {}
+    for key in ("grid_pred_decoded", "grid_pred_reg_decoded"):
+      res.update(("%s_%d" % (key, i), t) for i, t in enumerate(out[key]) if torch.is_tensor(t))
+    if out["beam_outputs"] is not None:
+      res.update(zip(("beam_logits", "beam_grid_ids", "beam_logprobs"), out["beam_outputs"]))
+    dump_outputs(dump_dir, res)
+    del out, res
   if use_graph:
     # graph replays do not pass through the C ABI's launch counter: count one launch-by-launch forward
     ops.reset_launch_count()

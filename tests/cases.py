@@ -156,3 +156,157 @@ def grad_sample_stride(size):
 
 
 ADV_SAMPLE_STRIDE = 7      # every 7th element of the augmented features is stored in simaug_multiview.npz
+
+
+# ---- reference-execution goldens (tests/golden/make_golden_refexec.py) --------------------------------------------
+REFEXEC_FORWARD = {
+    # name: oracle.default_config overrides, seed
+    "beam_k5_plain": ROLLOUTS["beam_k5_plain"],
+    "beam_k20_diverse": (dict(batch_size=3, use_grids=[False, True], use_beam_search=True, beam_size=20,
+                              diverse_beam=True, diverse_gamma=0.01, fix_num_timestep=1), 7),
+    "greedy_two_scale": (dict(batch_size=2, scene_h=24, scene_w=16), 8),
+    "no_gnn": (dict(batch_size=2, use_grids=[False, True], use_gnn=False), 9),
+}
+REFEXEC_TRAIN = (dict(batch_size=2, use_grids=[False, True]), 10,
+                 dict(grid_loss_weight=1.0, grid_reg_loss_weight=0.1, wd=0.001))
+SIMAUG_ATTACKS = ("fgsm", "pgd_mixup")
+FEED_DICT_CONFIGS = (dict(), dict(use_grids=[True, False]))
+
+
+def ref_sample(a, n=4096):
+  """Every k-th element of the flattened array, k the smallest stride that leaves at most n: what the
+  reference-execution goldens keep of a large output."""
+  a = np.asarray(a).reshape(-1)
+  return a[::max(1, -(-a.size // n))]
+
+
+def simaug_attack(mode, n, pred_len, eps, hw):
+  """Random target offsets and the (fgsm, step size, iterations, mixup beta) of a white_box_attack case."""
+  rng = np.random.default_rng(3)
+  off = rng.integers(1, hw, size=(n, pred_len)).astype(np.int32)
+  fgsm = mode == "fgsm"
+  step, iters, beta = (eps, 1, None) if fgsm else (0.03, 3, 0.4)
+  return off, fgsm, step, iters, beta
+
+
+def dropin_args(**kw):
+  """(argparse-like namespace for pred_models.get_model, synthetic config) at batch 3."""
+  import types
+  from multiverse_b200 import synthetic
+  cfg = synthetic.make_config(batch_size=3, **kw)
+  a = dict(vars(cfg))
+  a.update(modelname="m", runId=0, gpuid=0, use_soft_grid_class=False, soft_grid=1, use_gt_grid=False,
+           mask_grid_regression=False, use_single_decoder=False, use_teacher_forcing=False,
+           train_w_onehot=True, grid_loss_weight=1.0, grid_reg_loss_weight=0.1, wd=0.001, optimizer="adadelta")
+  return types.SimpleNamespace(**a), cfg
+
+
+def feed_digest(v):
+  """sha1 of the value as contiguous float64: equal digests and shapes <=> np.array_equal after the float64 cast."""
+  import hashlib
+  return hashlib.sha1(np.ascontiguousarray(np.asarray(v).astype(np.float64)).tobytes()).hexdigest()
+
+
+def feed_labels(model, feed):
+  """Placeholder -> the Model attribute holding it ("grid_obs_labels[1]"): placeholder names repeat across scales."""
+  labels = {}
+  for attr, v in vars(model).items():
+    for i, p in enumerate(v if isinstance(v, list) else [v]):
+      labels.setdefault(id(p), "%s[%d]" % (attr, i) if isinstance(v, list) else attr)
+  out = {labels[id(k)]: v for k, v in feed.items()}
+  assert len(out) == len(feed)
+  return out
+
+
+def put_feed_digests(d, prefix, model, feed):
+  feed = feed_labels(model, feed)
+  d[prefix + "names"] = np.asarray(sorted(feed))
+  for k, v in feed.items():
+    d[prefix + k + "/shape"] = np.asarray(np.asarray(v).shape, np.int64)
+    d[prefix + k + "/sha1"] = np.asarray(feed_digest(v))
+
+
+def check_feed_digests(g, prefix, model, feed):
+  """feed (placeholder -> value) holds, label for label, the stored values; returns the stored labels."""
+  feed = feed_labels(model, feed)
+  names = set(str(s) for s in g[prefix + "names"])
+  for name in names:
+    a = np.asarray(feed[name])
+    assert a.shape == tuple(g[prefix + name + "/shape"]), name
+    assert feed_digest(a) == str(g[prefix + name + "/sha1"]), name
+  return names
+
+
+def _dense_targets(traj, centers):
+  return [(np.asarray(t, np.float64)[:, None, None, :] - centers[None]).astype(np.float32) for t in traj]
+
+
+def put_batch(d, prefix, batch):
+  """A pred_utils batch (data lists, shared grid centres) as arrays.  The dense offset targets are not stored when
+  they equal float32(trajectory - cell centre), which load_batch then rebuilds."""
+  data, shared = batch.data, batch.shared
+  centers = {k: np.asarray(v) for k, v in shared.items() if k.startswith("grid_center_")}
+  for k, v in centers.items():
+    d[prefix + "shared/" + k] = v
+  for k, v in data.items():
+    if k.startswith(("obs_grid_target_all_", "pred_grid_target_all_")):
+      j = k.rsplit("_", 1)[1]
+      traj = data["obs_traj" if k.startswith("obs") else "pred_traj"]
+      if all(np.array_equal(a, b) for a, b in zip(_dense_targets(traj, centers["grid_center_" + j]), v)):
+        d[prefix + "rebuilt/" + k] = np.asarray(len(v))
+        continue
+    kind = "list/" if isinstance(v, list) else ("array/" if isinstance(v, np.ndarray) else "scalar/")
+    d[prefix + kind + k] = np.stack([np.asarray(a) for a in v]) if kind == "list/" else np.asarray(v)
+
+
+def load_batch(g, prefix):
+  import types
+  data, shared, rebuilt = {}, {}, []
+  for key in g.files:
+    if not key.startswith(prefix):
+      continue
+    kind, k = key[len(prefix):].split("/", 1)
+    if kind == "shared":
+      shared[k] = g[key]
+    elif kind == "list":
+      data[k] = list(g[key])
+    elif kind == "array":
+      data[k] = g[key]
+    elif kind == "scalar":
+      data[k] = g[key].item()
+    elif kind == "rebuilt":
+      rebuilt.append(k)
+  for k in rebuilt:
+    traj = data["obs_traj" if k.startswith("obs") else "pred_traj"]
+    data[k] = _dense_targets(traj, shared["grid_center_" + k.rsplit("_", 1)[1]])
+  return types.SimpleNamespace(data=data, shared=shared)
+
+
+def multiview_feed_case(pm):
+  """A multiview_train batch (3 samples, 3 extra views) and the drop-in Model it is fed to.  Returns
+  (args, config, model, batch)."""
+  import types
+  args, cfg = dropin_args(use_grids=[False, True])
+  n, m = args.batch_size, 3
+  args.is_train, args.multiview_train, args.multiview_max_num, args.multiview_exp = True, True, m, 1
+  model = pm.get_model(args, gpuid=0)
+  rng = np.random.default_rng(5)
+  t_in, t_pred = cfg.obs_len, cfg.pred_len
+
+  def views(count):
+    return [np.stack([rng.integers(0, h * w, count) for (h, w) in cfg.scene_grids]) for _ in range(m)]
+  data = dict(obs_grid_class=[np.stack([rng.integers(0, h * w, t_in) for (h, w) in cfg.scene_grids]) for _ in range(n)],
+              pred_grid_class=[np.stack([rng.integers(0, h * w, t_pred) for (h, w) in cfg.scene_grids]) for _ in range(n)],
+              batch_scene_feat=rng.random((7, cfg.scene_h, cfg.scene_w, cfg.scene_class)).astype(np.float32),
+              batch_obs_scene=rng.integers(0, 7, (n, t_in, 1)),
+              batch_extra_obs_scene=rng.integers(0, 7, (n, m, t_in, 1)), extra=[])
+  for j, (h, w) in enumerate(cfg.scene_grids):
+    data["obs_grid_target_all_%d" % j] = [rng.standard_normal((t_in, h, w, 2)).astype(np.float32) for _ in range(n)]
+    data["pred_grid_target_all_%d" % j] = [rng.standard_normal((t_pred, h, w, 2)).astype(np.float32) for _ in range(n)]
+  for i in range(n):
+    ex = dict(obs_grid_class=views(t_in), pred_grid_class=views(t_pred))
+    for j, (h, w) in enumerate(cfg.scene_grids):
+      ex["obs_grid_target_all_%d" % j] = [rng.standard_normal((t_in, h, w, 2)).astype(np.float32) for _ in range(m)]
+      ex["pred_grid_target_all_%d" % j] = [rng.standard_normal((t_pred, h, w, 2)).astype(np.float32) for _ in range(m)]
+    data["extra"].append(ex)
+  return args, cfg, model, types.SimpleNamespace(data=data)

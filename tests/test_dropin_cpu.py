@@ -2,11 +2,8 @@
 """CPU tests of the drop-in boundary (host logic only - no kernel runs here).
 
 With multiverse_b200/dropin first on sys.path the reference's callers import OUR `pred_models`
-and the `tensorflow`-named shim.  When the reference tree is mounted (this container; it does not
-exist on the GPU box) its unchanged code/test.py flow and its own Model.get_feed_dict are run
-against ours."""
-import importlib
-import importlib.util
+and the `tensorflow`-named shim.  The reference's own Model.get_feed_dict results are stored in
+tests/golden/refexec_feed_dicts.npz (tests/golden/make_golden_refexec.py)."""
 import os
 import sys
 import types
@@ -16,14 +13,9 @@ import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DROPIN = os.path.join(ROOT, "multiverse_b200", "dropin")
-REF = "/root/reference/code"
-have_ref = os.path.exists(os.path.join(REF, "pred_utils.py"))
-
-
-def as_host(out, wanted):
-  """Model._engine_forward's contract: {(fetch name, index): numpy array (or [] for an unused scale)}."""
-  conv = lambda t: t.numpy() if hasattr(t, "numpy") else t
-  return {k: conv(out[k[0]][k[1]]) for k in wanted}
+sys.path.insert(0, os.path.join(ROOT, "tests"))
+import cases  # noqa: E402
+FEED_GOLD = os.path.join(ROOT, "tests", "golden", "refexec_feed_dicts.npz")
 
 
 @pytest.fixture()
@@ -40,13 +32,7 @@ def dropin(monkeypatch):
 
 
 def make_args(tmp_path, **kw):
-  from multiverse_b200 import synthetic
-  cfg = synthetic.make_config(batch_size=3, **kw)
-  a = dict(vars(cfg))
-  a.update(modelname="m", runId=0, gpuid=0, use_soft_grid_class=False, soft_grid=1, use_gt_grid=False,
-           mask_grid_regression=False, use_single_decoder=False, use_teacher_forcing=False,
-           train_w_onehot=True, grid_loss_weight=1.0, grid_reg_loss_weight=0.1, wd=0.001, optimizer="adadelta")
-  return types.SimpleNamespace(**a), cfg
+  return cases.dropin_args(**kw)
 
 
 def test_model_surface_matches_reference_names(dropin, tmp_path):
@@ -128,245 +114,41 @@ def test_saver_relative_path_round_trip(dropin, tmp_path, monkeypatch):
   assert os.path.exists(st2.model_checkpoint_path + ".npz")
 
 
-@pytest.mark.skipif(not have_ref, reason="reference tree not mounted")
-def test_get_feed_dict_equals_the_references(dropin, tmp_path, monkeypatch):
+def test_get_feed_dict_equals_the_references(dropin, tmp_path):
   """Our vectorised Model.get_feed_dict against the reference's own method
-  (code/pred_models.py:1042-1194) executed on our Model instance."""
+  (code/pred_models.py:1042-1194) executed on our Model instance, on the batches code/pred_utils.py
+  made of synthetic.write_npz(.., 5, seed=3) - both stored in tests/golden/refexec_feed_dicts.npz."""
   tf, pm = dropin
-  from multiverse_b200 import synthetic
-  monkeypatch.syspath_prepend(REF)
-  spec = importlib.util.spec_from_file_location("ref_pred_models", os.path.join(REF, "pred_models.py"))
-  ref = importlib.util.module_from_spec(spec)
-  spec.loader.exec_module(ref)
-  import pred_utils
-  for kw in (dict(), dict(use_grids=[True, False])):
+  g = np.load(FEED_GOLD)
+  for c, kw in enumerate(cases.FEED_DICT_CONFIGS):
     tf.reset_default_graph()
     args, cfg = make_args(tmp_path, **kw)
-    args.prepropath = str(tmp_path)
-    synthetic.write_npz(str(tmp_path / "data_test.npz"), cfg, 5, seed=3)
-    data = pred_utils.read_data(args, "test")
     model = pm.get_model(args, gpuid=0)
-    for is_train in (False, True):
-      for _, batch in data.get_batches(args.batch_size, full=True, shuffle=False):
-        theirs = ref.Model.get_feed_dict(model, batch, is_train=is_train)
+    for b in range(2):
+      batch = cases.load_batch(g, "cfg%d/batch%d/" % (c, b))
+      for is_train in (False, True):
         args.device_grid_feeds = False           # the reference's feed dict, key for key
         ours = model.get_feed_dict(batch, is_train=is_train)
-        assert set(ours) == set(theirs)
-        for k in theirs:
-          a, b = np.asarray(ours[k]), np.asarray(theirs[k])
-          assert a.shape == b.shape, k
-          assert np.array_equal(a.astype(np.float64), b.astype(np.float64)), k
+        assert cases.check_feed_digests(g, "cfg%d/batch%d/train%d/" % (c, b, is_train), model, ours) == \
+            set(cases.feed_labels(model, ours))
         # row f-1 (default): the dense offsets are replaced by the trajectories + cell centres they came from
         args.device_grid_feeds = True
         compact = model.get_feed_dict(batch, is_train=is_train)
         used = [j for j in range(2) if args.use_grids[j]]
         if is_train:
-          assert set(compact) == set(theirs)     # training keeps the dense path
+          assert set(compact) == set(ours)       # training keeps the dense path
           continue
         assert model.obs_traj in compact and all(model.grid_obs_regress[j] not in compact for j in used)
         n_have = len(batch.data["obs_traj"])
         for j in used:
           dense = (compact[model.obs_traj][:, :, None, None, :] - compact[model.grid_centers[j]][None, None]).astype(np.float32)
-          assert np.array_equal(dense[:n_have], np.asarray(theirs[model.grid_obs_regress[j]], np.float32)[:n_have])
+          assert np.array_equal(dense[:n_have], np.asarray(ours[model.grid_obs_regress[j]], np.float32)[:n_have])
         small = compact[model.obs_traj].nbytes + sum(compact[model.grid_centers[j]].nbytes for j in used)
-        big = sum(np.asarray(theirs[model.grid_obs_regress[j]], np.float32).nbytes for j in used)
+        big = sum(np.asarray(ours[model.grid_obs_regress[j]], np.float32).nbytes for j in used)
         assert small < big / 4        # (at batch 4; the centres are per model, the trajectories 128 B per row)
     # a batch whose dense targets do not come from its trajectories keeps the dense path
     batch.data["obs_grid_target_all_0"] = [a + 1.0 for a in batch.data["obs_grid_target_all_0"]]
     assert model.obs_traj not in model.get_feed_dict(batch, is_train=False)
-
-
-@pytest.mark.skipif(not have_ref, reason="reference tree not mounted")
-def test_reference_test_py_flow_runs_unchanged(dropin, tmp_path, monkeypatch, capsys):
-  """code/test.py (byte-identical) imported and driven end to end - argparse, process_args,
-  read_data, get_model, initialize(load) through our Saver, Tester, evaluate and the metric
-  print-out - with the device forward stubbed out (there is no GPU in this container)."""
-  tf, pm = dropin
-  from multiverse_b200 import synthetic
-  import multiverse_b200.pred_models as impl
-  monkeypatch.syspath_prepend(REF)
-  cfg = synthetic.make_config(batch_size=4, use_grids=[True, False])
-  prepro = tmp_path / "prepro"; prepro.mkdir()
-  synthetic.write_npz(str(prepro / "data_test.npz"), cfg, 6, seed=4)
-  argv = ["test.py", str(prepro), str(tmp_path / "out"), "modelname", "--runId", "0", "--load_best",
-          "--is_baseline" if False else "--use_scene_enc", "--use_gnn", "--scene_h", "72", "--scene_w", "36",
-          "--scene_grid_strides", "2,4", "--use_grids", "1,0", "--batch_size", "4", "--emb_size", "32",
-          "--scene_conv_dim", "64", "--scene_class", "11", "--activation_func", "tanh", "--obs_len", "8",
-          "--pred_len", "12", "--convlstm_kernel", "3", "--enc_hidden_size", "256", "--dec_hidden_size", "256"]
-  monkeypatch.setattr(sys, "argv", argv)
-  spec = importlib.util.spec_from_file_location("ref_test", os.path.join(REF, "test.py"))
-  ref_test = importlib.util.module_from_spec(spec)
-  spec.loader.exec_module(ref_test)
-  import pred_utils
-  args = ref_test.parser.parse_args()
-  args.is_train, args.is_test = False, True
-  args = pred_utils.process_args(args)
-  assert args.scene_grids == [(36, 18), (18, 9)]
-
-  # a "trained" checkpoint in the location test.py --load_best expects
-  model0 = pm.get_model(args, gpuid=0)
-  tf.global_variables_initializer().run()
-  tf.train.Saver().save(tf.Session(), args.save_dir_best_model, global_step=model0.global_step)
-  tf.reset_default_graph()
-
-  calls = []
-
-  def fake_forward(self, feed, wanted):
-    import torch
-    n, tp = self.N, self.config.pred_len
-    calls.append(feed)
-    out = dict(grid_pred_decoded=[], grid_pred_reg_decoded=[], beam_outputs=None)
-    for i, (h, w) in enumerate(self.config.scene_grids):
-      if not self.config.use_grids[i]:
-        out["grid_pred_decoded"].append([]); out["grid_pred_reg_decoded"].append([])
-      else:
-        out["grid_pred_decoded"].append(torch.zeros(n, tp, h, w, 1))
-        out["grid_pred_reg_decoded"].append(torch.zeros(n, tp, h, w, 2))
-    return as_host(out, wanted)
-
-  monkeypatch.setattr(impl.Model, "_engine_forward", fake_forward)
-  ref_test.main(args)
-  text = capsys.readouterr().out
-  assert "total test samples:6" in text and "grid0_traj_ade" in text
-  assert len(calls) == 2                                  # ceil(6 / 4) batches
-  assert calls[0][[k for k in calls[0] if getattr(k, "name", "") == "scene_feat"][0]].shape[1:] == (72, 36, 11)
-
-
-@pytest.mark.skipif(not have_ref, reason="reference tree not mounted")
-def test_reference_train_py_flow_runs_unchanged(dropin, tmp_path, monkeypatch, capsys):
-  """code/train.py (byte-identical): argparse -> process_args -> read_data -> get_model -> Trainer /
-  Tester -> the training loop with periodic save + evaluate, on our surface; the device work
-  (Model._train_step / _engine_forward) is stubbed because this container has no GPU."""
-  tf, pm = dropin
-  from multiverse_b200 import synthetic
-  import multiverse_b200.pred_models as impl
-  monkeypatch.syspath_prepend(REF)
-  cfg = synthetic.make_config(batch_size=4, use_grids=[True, False])
-  prepro = tmp_path / "prepro"; prepro.mkdir()
-  synthetic.write_npz(str(prepro / "data_train.npz"), cfg, 10, seed=5)
-  synthetic.write_npz(str(prepro / "data_val.npz"), cfg, 6, seed=6)
-  argv = ["train.py", str(prepro), str(tmp_path / "out"), "modelname", "--runId", "0", "--use_scene_enc", "--use_gnn",
-          "--scene_h", "72", "--scene_w", "36", "--scene_grid_strides", "2,4", "--use_grids", "1,0",
-          "--batch_size", "4", "--emb_size", "32", "--scene_conv_dim", "64", "--scene_class", "11",
-          "--activation_func", "tanh", "--obs_len", "8", "--pred_len", "12", "--train_w_onehot", "--wd", "0.001",
-          "--num_epochs", "2", "--save_period", "3", "--init_lr", "0.3", "--grid_reg_loss_weight", "0.2",
-          "--val_grid_num", "0"]
-  monkeypatch.setattr(sys, "argv", argv)
-  spec = importlib.util.spec_from_file_location("ref_train", os.path.join(REF, "train.py"))
-  ref_train = importlib.util.module_from_spec(spec)
-  spec.loader.exec_module(ref_train)
-  import pred_utils
-  args = ref_train.parser.parse_args()
-  args.is_train = True
-  args.is_test = False
-  args = pred_utils.process_args(args)
-  steps = []
-
-  def fake_train_step(self, feed, apply=True):
-    steps.append(int(self.global_step.value))
-    self.global_step.value = np.asarray(int(self.global_step.value) + 1, dtype="int32")
-    lr = self.learning_rate(steps[-1])
-    assert abs(lr - 0.3 * 0.95 ** (steps[-1] // int(10 / 4 * 2.0))) < 1e-12      # staircase decay, :1656-1665
-    return dict(loss=np.float32(1.0 / (1 + len(steps))), wd_loss=np.float32(0.1), train_op=None,
-                classification_loss={0: np.float32(0.5)}, regression_loss={0: np.float32(0.4)})
-
-  def fake_forward(self, feed, wanted):
-    import torch
-    n, tp = self.N, self.config.pred_len
-    out = dict(grid_pred_decoded=[], grid_pred_reg_decoded=[], beam_outputs=None)
-    for i, (h, w) in enumerate(self.config.scene_grids):
-      ok = self.config.use_grids[i]
-      out["grid_pred_decoded"].append(torch.zeros(n, tp, h, w, 1) if ok else [])
-      out["grid_pred_reg_decoded"].append(torch.zeros(n, tp, h, w, 2) if ok else [])
-    return as_host(out, wanted)
-
-  monkeypatch.setattr(impl.Model, "_train_step", fake_train_step)
-  monkeypatch.setattr(impl.Model, "_engine_forward", fake_forward)
-  ref_train.main(args)
-  text = capsys.readouterr().out
-  assert steps == list(range(6))                       # ceil(10/4) * 2 epochs
-  assert "best eval on val grid0_traj_ade" in text
-  ck = tf.train.get_checkpoint_state(args.save_dir)
-  assert ck is not None and os.path.exists(ck.model_checkpoint_path + ".npz")
-  assert tf.train.get_checkpoint_state(args.save_dir_best) is not None
-
-
-@pytest.mark.skipif(not have_ref, reason="reference tree not mounted")
-def test_reference_multifuture_inference_pieces_run_unchanged(dropin, tmp_path, monkeypatch):
-  """code/multifuture_inference.py (byte-identical): its PredictionModelInference subclass of OUR Model,
-  its Namespace config (:419-452), load_model_weights (:275-299) through our Saver, its own
-  get_feed_dict (:304-385) and the fetch list of :462-472 - the device forward is stubbed."""
-  tf, pm = dropin
-  from multiverse_b200 import synthetic
-  import multiverse_b200.pred_models as impl
-  import argparse
-  monkeypatch.syspath_prepend(REF)
-  monkeypatch.setattr(sys, "argv", ["multifuture_inference.py", "a", "b", "c", "d"])
-  spec = importlib.util.spec_from_file_location("ref_mfi", os.path.join(REF, "multifuture_inference.py"))
-  mfi = importlib.util.module_from_spec(spec)
-  spec.loader.exec_module(mfi)                      # __main__ guard: only definitions run
-  args = mfi.parser.parse_args(["traj", "mf", "model", "out.p", "--num_out", "20", "--diverse_beam",
-                                "--diverse_gamma", "0.01", "--fix_num_timestep", "1", "--use_gnn",
-                                "--use_scene_enc", "--emb_size", "32", "--scene_h", "72", "--scene_w", "36"])
-  mfi.add_grid(args)
-  assert args.scene_grids == [(36, 18), (18, 9)] and args.use_grids == [True, False]
-  args.use_beam_search = True
-  model_config = argparse.Namespace(
-      modelname="model", batch_size=1, beam_size=args.num_out, use_beam_search=args.use_beam_search,
-      diverse_beam=args.diverse_beam, diverse_gamma=args.diverse_gamma, fix_num_timestep=args.fix_num_timestep,
-      use_teacher_forcing=False, is_train=False, scene_h=args.scene_h, scene_w=args.scene_w,
-      scene_class=args.scene_class, use_soft_grid_class=args.use_soft_grid_class,
-      use_single_decoder=args.use_single_decoder, pred_len=12, emb_size=args.emb_size,
-      enc_hidden_size=args.enc_hidden_size, dec_hidden_size=args.dec_hidden_size, activation_func=tf.nn.tanh,
-      scene_conv_kernel=args.scene_conv_kernel, use_scene_enc=args.use_scene_enc,
-      scene_conv_dim=args.scene_conv_dim, convlstm_kernel=args.convlstm_kernel, use_gnn=args.use_gnn,
-      keep_prob=1.0, scene_grid_strides=args.scene_grid_strides, scene_grids=args.scene_grids,
-      use_grids=args.use_grids)
-  # a checkpoint of the same architecture, written through the shim Saver
-  cfg = synthetic.make_config(batch_size=1, use_grids=[True, False])
-  donor_args = types.SimpleNamespace(**vars(cfg)); donor_args.modelname = "donor"
-  donor_args.use_soft_grid_class = False
-  donor = pm.get_model(donor_args, gpuid=0)
-  tf.global_variables_initializer().run()
-  want = {k: v.copy() for k, v in donor.weights().items()}
-  tf.train.Saver().save(tf.Session(), str(tmp_path / "ckpt" / "save"), global_step=7)
-  tf.reset_default_graph()
-
-  with tf.Session() as sess:
-    with tf.device("/gpu:0"):
-      model = mfi.PredictionModelInference(model_config, model_config.modelname)
-    mfi.load_model_weights(str(tmp_path / "ckpt"), sess, top_scope="person_pred")
-    for k, v in model.weights().items():
-      assert np.array_equal(v, want[k]), k
-    # inputs in the layout get_inputs (:158-272) produces, for 2 trajectories with 12 / 17 future steps
-    f = synthetic.make_feeds(cfg, 2, 3)
-    inputs = dict(obs_grid_class=[np.stack([f["grid_obs_labels"][j][i] for j in range(2)]) for i in range(2)],
-                  obs_grid_target=[[f["grid_obs_regress"][j][i] for j in range(2)] for i in range(2)],
-                  obs_scene=[np.full((8, 1), i, dtype="int32") for i in range(2)],
-                  scene_feats=f["scene_feat"], max_pred_lengths=[12, 17])
-    seen = []
-
-    def fake_forward(self, feed, wanted):
-      import torch
-      tp = self._fed_pred_len(feed)
-      seen.append(tp)
-      h, w = self.config.scene_grids[0]
-      return as_host(dict(grid_pred_decoded=[torch.zeros(1, tp, h, w, 1), []],
-                          grid_pred_reg_decoded=[torch.zeros(1, tp, h, w, 2), []],
-                          beam_outputs=[torch.zeros(1, 20, tp, h * w), torch.zeros(1, 20, tp, dtype=torch.int32),
-                                        torch.zeros(1, 20)]), wanted)
-
-    monkeypatch.setattr(impl.Model, "_engine_forward", fake_forward)
-    for i in range(2):
-      feed_dict = model.get_feed_dict(inputs, args, i)
-      assert feed_dict[model.scene_feat].shape == (1, 72, 36, 11)
-      output_tensors = [model.grid_pred_decoded[0], model.grid_pred_reg_decoded[0], model.beam_outputs]
-      class_output, reg_output, beam_outputs = sess.run(output_tensors, feed_dict=feed_dict)
-      pred_len = inputs["max_pred_lengths"][i]
-      assert reg_output.reshape([1, pred_len, -1, 2]).shape[2] == 36 * 18      # :479
-      beam_logits, beam_grid_ids, beam_logprobs = beam_outputs
-      assert beam_grid_ids.shape == (1, 20, pred_len) and beam_logits.shape == (1, 20, pred_len, 648)
-    assert seen == [12, 17]          # the rollout length follows the FED pred_length, not config.pred_len
 
 
 def test_tf_checkpoint_bundle_reader(dropin, tmp_path):
@@ -611,56 +393,21 @@ def test_session_run_leaves_no_reference_cycle_on_the_results(monkeypatch):
     gc.enable()
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/SimAug/code/pred_models.py"), reason="reference tree not mounted")
-def test_multiview_feed_dict_equals_simaugs(dropin, tmp_path, monkeypatch):
+def test_multiview_feed_dict_equals_simaugs(dropin, tmp_path):
   """The extra-view feeds of a multiview_train batch (obs_scene_extra, grid_*_extra) against SimAug's own
-  Model.get_feed_dict (SimAug/code/pred_models.py:1457-1560) executed on our Model instance, key for key on every
-  placeholder that method fills."""
+  Model.get_feed_dict (SimAug/code/pred_models.py:1457-1560) executed on our Model instance (stored in
+  tests/golden/refexec_feed_dicts.npz), key for key on every placeholder that method fills."""
   tf, pm = dropin
-  import types
-  monkeypatch.syspath_prepend(os.path.join(ROOT, "oracle", "tf1_eager"))
-  spec = importlib.util.spec_from_file_location("ref_simaug_pred_models", "/root/reference/SimAug/code/pred_models.py")
-  saved = sys.modules.get("tensorflow")
-  ref = importlib.util.module_from_spec(spec)
-  spec.loader.exec_module(ref)                    # binds `tf` to whatever `tensorflow` is importable: only numpy is used below
-  if saved is not None:
-    sys.modules["tensorflow"] = saved
   tf.reset_default_graph()
-  args, cfg = make_args(tmp_path, use_grids=[False, True])
-  n, m = args.batch_size, 3
-  args.is_train, args.multiview_train, args.multiview_max_num, args.multiview_exp = True, True, m, 1
-  model = pm.get_model(args, gpuid=0)
-  rng = np.random.default_rng(5)
+  args, cfg, model, batch = cases.multiview_feed_case(pm)
   ns = len(cfg.scene_grids)
-  t_in, t_pred = cfg.obs_len, cfg.pred_len
-  def views(count):
-    return [np.stack([rng.integers(0, h * w, count) for (h, w) in cfg.scene_grids]) for _ in range(m)]
-  data = dict(obs_grid_class=[np.stack([rng.integers(0, h * w, t_in) for (h, w) in cfg.scene_grids]) for _ in range(n)],
-              pred_grid_class=[np.stack([rng.integers(0, h * w, t_pred) for (h, w) in cfg.scene_grids]) for _ in range(n)],
-              batch_scene_feat=rng.random((7, cfg.scene_h, cfg.scene_w, cfg.scene_class)).astype(np.float32),
-              batch_obs_scene=rng.integers(0, 7, (n, t_in, 1)),
-              batch_extra_obs_scene=rng.integers(0, 7, (n, m, t_in, 1)), extra=[])
-  for j, (h, w) in enumerate(cfg.scene_grids):
-    data["obs_grid_target_all_%d" % j] = [rng.standard_normal((t_in, h, w, 2)).astype(np.float32) for _ in range(n)]
-    data["pred_grid_target_all_%d" % j] = [rng.standard_normal((t_pred, h, w, 2)).astype(np.float32) for _ in range(n)]
-  for i in range(n):
-    ex = dict(obs_grid_class=views(t_in), pred_grid_class=views(t_pred))
-    for j, (h, w) in enumerate(cfg.scene_grids):
-      ex["obs_grid_target_all_%d" % j] = [rng.standard_normal((t_in, h, w, 2)).astype(np.float32) for _ in range(m)]
-      ex["pred_grid_target_all_%d" % j] = [rng.standard_normal((t_pred, h, w, 2)).astype(np.float32) for _ in range(m)]
-    data["extra"].append(ex)
-  batch = types.SimpleNamespace(data=data)
-  theirs = ref.Model.get_feed_dict(model, batch, is_train=True)
   ours = model.get_feed_dict(batch, is_train=True)
-  assert set(theirs) <= set(ours)
+  theirs = cases.check_feed_digests(np.load(FEED_GOLD), "multiview/", model, ours)     # theirs <= ours, values equal
   extra_keys = [model.obs_scene_extra] + [p for j in range(ns) if cfg_use(args, j) for p in
                                           (model.grid_obs_labels_extra[j], model.grid_pred_labels_T_extra[j],
                                            model.grid_pred_regress_extra[j], model.grid_obs_regress_extra[j])]
-  assert all(k in theirs for k in extra_keys)
-  for k in theirs:
-    a, b = np.asarray(ours[k]), np.asarray(theirs[k])
-    assert a.shape == b.shape, k
-    assert np.array_equal(a.astype(np.float64), b.astype(np.float64)), k
+  labels = cases.feed_labels(model, {k: None for k in extra_keys})
+  assert set(labels) <= theirs
 
 
 def cfg_use(args, j):

@@ -1,10 +1,10 @@
 # coding=utf-8
 """SURVEY.md section 8 row f-4, the pin: SimAug's multi-view augmentation as EXECUTED FROM THE REFERENCE'S OWN FILE
-(unmodified /root/reference/SimAug/code/pred_models.py on the eager TF-1.15 stand-in, oracle/tf1_eager/run_simaug.py)
-against (a) the committed golden tests/golden/simaug_multiview.npz and (b) the same pipeline written on the oracle
+(the unmodified SimAug/code/pred_models.py of the original project on the eager TF-1.15 stand-in,
+oracle/tf1_eager/run_simaug.py; stored by tests/golden/make_golden_refexec.py in tests/golden/refexec_simaug.npz, the
+augmented features as an fp64 sample, cases.ref_sample) against the same pipeline written on the oracle
 (oracle/multiverse_ref_torch.py: autograd input gradient, per-view losses, selection, mixup, mixed-label objective) -
-the expectation the GPU tests of multiverse_b200/simaug.py and TrainEngine's mixup path are held to.
-Skipped where /root/reference does not exist (the GPU box)."""
+the expectation the GPU tests of multiverse_b200/simaug.py and TrainEngine's mixup path are held to."""
 import os
 import sys
 
@@ -17,10 +17,15 @@ sys.path.insert(0, os.path.join(ROOT, "tests"))
 import cases  # noqa: E402
 from oracle import multiverse_ref as R  # noqa: E402
 from oracle import multiverse_ref_torch as RT  # noqa: E402
-from oracle.tf1_eager import run_simaug as RS  # noqa: E402
 
-pytestmark = pytest.mark.skipif(not RS.available(), reason="needs /root/reference (not on the GPU box)")
-GOLD = os.path.join(ROOT, "tests", "golden", "simaug_multiview.npz")
+GOLD = os.path.join(ROOT, "tests", "golden", "refexec_simaug.npz")
+
+
+def sampled(a, g, key):
+  """The stored sample's positions of a (whose shape must be the reference array's)."""
+  a = np.asarray(a, np.float64)
+  assert a.shape == tuple(g[key + "/shape"]), key
+  return cases.ref_sample(a, 16384)
 
 
 def oracle_pipeline(exp):
@@ -71,38 +76,33 @@ def oracle_pipeline(exp):
 
 @pytest.mark.parametrize("exp", [1, 4, 3])
 def test_reference_execution_matches_golden_and_oracle_pipeline(exp):
-  cfg, w, f, extra, spec = cases.simaug_case()
-  rcfg = R.default_config(**spec["config"])
-  ref = RS.multiview(rcfg, w, f, extra, spec["m"], exp, spec["eps"], spec["beta_draw"], with_trainer=(exp == 3),
-                     double_weighting=(exp == 3))
   g = np.load(GOLD)
-  assert str(g["source"]).startswith("reference_exec")
-  samp = ref["adv_final"].reshape(-1)[::cases.ADV_SAMPLE_STRIDE]
-  assert np.abs(samp - g["exp%d_adv_final_sample" % exp]).max() < 1e-6
-  assert abs(ref["beta_weight"] - float(g["exp%d_beta" % exp])) < 1e-12
-  assert np.abs(np.array(ref["losses"]) - g["exp%d_losses" % exp]).max() < 1e-9
-  # ---- the oracle's pipeline
+  p = "exp%d/" % exp
   o = oracle_pipeline(exp)
-  assert abs(o["beta"] - ref["beta_weight"]) < 1e-12
-  d = np.abs(o["adv_final"] - ref["adv_final"])
+  assert abs(o["beta"] - float(g[p + "beta"])) < 1e-12
+  d = np.abs(sampled(o["adv_final"], g, p + "adv_final") - g[p + "adv_final"])
   # both are fp64: the sign of an input-gradient entry that is ~0 is the only thing that may differ
-  assert (d <= 1e-9).mean() > 0.99999 and d.max() <= 2 * spec["eps"] + 1e-9
-  assert np.abs(np.array(o["losses"]) - np.array(ref["losses"])).max() < 1e-6 * max(ref["losses"])
+  assert (d <= 1e-9).mean() > 0.99999 and d.max() <= 2 * cases.simaug_case()[4]["eps"] + 1e-9
+  ref_losses = g[p + "losses"]
+  assert np.abs(np.array(o["losses"]) - ref_losses).max() < 1e-6 * max(ref_losses)
   if exp == 3:
-    assert np.array_equal(o["selected"], ref["selected_extra_indices"])
-    assert np.abs(o["focal"] - ref["focal_loss_weight"]).max() < 1e-9
+    assert np.array_equal(o["selected"], g[p + "selected"])
+    assert np.abs(o["focal"] - g[p + "focal"]).max() < 1e-9
     worst = 0.0
-    for k, gr in ref["grads"].items():
-      og = o["grads"][k]
-      scale = max(np.abs(gr).max(), 1e-30)
-      worst = max(worst, np.abs(og - gr).max() / scale)
-      samp_g = gr.reshape(-1)[::cases.grad_sample_stride(gr.size)]
-      assert np.abs(samp_g - g["exp3_grad_sample/" + k]).max() <= 1e-6 * scale + 1e-12, k
-    print("exp 3: oracle vs reference-exec gradients, worst relative error %.2e over %d variables" % (worst, len(ref["grads"])))
+    names = set(k[len(p + "grad/"):] for k in g.files
+                if k.startswith(p + "grad/") and not k.endswith(("/shape", "/absmax")))
+    assert names and names <= set(o["grads"])
+    for k in names:
+      key = p + "grad/" + k
+      og = np.asarray(o["grads"][k], np.float64)
+      assert og.shape == tuple(g[key + "/shape"]), k
+      scale = max(float(g[key + "/absmax"]), 1e-30)
+      worst = max(worst, np.abs(cases.ref_sample(og, 1024) - g[key]).max() / scale)
+    print("exp 3: oracle vs reference-exec gradients, worst relative error %.2e over %d variables" % (worst, len(names)))
     assert worst < 1e-6
 
 
-@pytest.mark.parametrize("mode", ["fgsm", "pgd_mixup"])
+@pytest.mark.parametrize("mode", cases.SIMAUG_ATTACKS)
 def test_white_box_attack_reference_execution_matches_oracle_pipeline(mode):
   """white_box_attack (SimAug/code/pred_models.py:60-170) as executed from the reference file - targeted FGSM, and PGD
   (tf.while_loop, 3 iterations, bounds around the clean input) followed by the mixup with the clean input - against
@@ -110,14 +110,11 @@ def test_white_box_attack_reference_execution_matches_oracle_pipeline(mode):
   white_box_attack and mvb_adv_step / mvb_mix implement (GPU: test_simaug_scene_input_gradient_and_attack)."""
   cfg, w, f, extra, spec = cases.simaug_case()
   rcfg = R.default_config(**spec["config"])
+  g = np.load(GOLD)
   n, eps, hw = spec["n"], spec["eps"], 18 * 9
-  rng = np.random.default_rng(3)
-  off = rng.integers(1, hw, size=(n, cfg.pred_len)).astype(np.int32)
-  fgsm = mode == "fgsm"
-  step, iters, beta = (eps, 1, None) if fgsm else (0.03, 3, 0.4)
-  ref = RS.adversarial(rcfg, w, f, eps, off, fgsm=fgsm, step_size=step, num_iter=iters, mixup_beta=beta)
+  off, fgsm, step, iters, beta = cases.simaug_attack(mode, n, cfg.pred_len, eps, hw)
   target = (f["grid_pred_labels"][1].astype(np.int64) + off) % hw                       # create_random_target
-  assert np.array_equal(ref["target_label"], target) and not (target == f["grid_pred_labels"][1]).any()
+  assert np.array_equal(g[mode + "/target_label"], target) and not (target == f["grid_pred_labels"][1]).any()
   # the oracle's pipeline: one private frame per (sample, step) row, like the reference's [N*T,SH,SW,SC] input
   t_obs = cfg.obs_len
   x = f["scene_feat"].astype(np.float64)[f["obs_scene"]].reshape((n * t_obs,) + f["scene_feat"].shape[1:])
@@ -125,13 +122,14 @@ def test_white_box_attack_reference_execution_matches_oracle_pipeline(mode):
   lo, hi = np.clip(x - eps, -1, 1), np.clip(x + eps, -1, 1)
   adv = x.copy()
   for _ in range(iters):
-    g = RT.scene_input_grad(rcfg, w, dict(rows, scene_feat=adv), target, 1)
-    adv = np.minimum(np.maximum(adv - step * np.sign(g), lo), hi)
+    gr = RT.scene_input_grad(rcfg, w, dict(rows, scene_feat=adv), target, 1)
+    adv = np.minimum(np.maximum(adv - step * np.sign(gr), lo), hi)
   if beta is not None:
     adv = x * beta + adv * (1 - beta)
-  d = np.abs(adv - ref["adv_final"])
-  print("white_box_attack %s: %.6f of the pixels equal, max diff %.3g" % (mode, (d <= 1e-9).mean(), d.max()))
+  d = np.abs(sampled(adv, g, mode + "/adv_final") - g[mode + "/adv_final"])
+  print("white_box_attack %s: %.6f of the sampled pixels equal, max diff %.3g" % (mode, (d <= 1e-9).mean(), d.max()))
   assert (d <= 1e-9).mean() > 0.9999 and d.max() <= 2 * eps + 1e-9
-  # and the training tower on the attacked features
-  _, losses, _, _ = RT.loss_and_grads(rcfg, w, dict(rows, scene_feat=ref["adv_final"]))
-  assert np.abs(np.array(losses) - np.array(ref["losses"])).max() < 1e-9 * max(ref["losses"])
+  # and the training tower on the attacked features: the oracle's losses on its own attacked features
+  _, losses, _, _ = RT.loss_and_grads(rcfg, w, dict(rows, scene_feat=adv))
+  ref_losses = g[mode + "/losses"]
+  assert np.abs(np.array(losses) - ref_losses).max() < 1e-9 * max(ref_losses)
