@@ -19,6 +19,19 @@ CELL_CASES = {
 }
 
 
+def cell_inputs(ns, h, w, cx, seed, x_scale=1.0):
+  """Seeded ConvLSTM cell inputs of any size, drawn like cell_case: Glorot-range kernel, small biases, x of the
+  given scale, tanh-bounded h and unit-scale c (tests/test_cell_variants_gpu.py and its worker process)."""
+  rng = np.random.default_rng(seed)
+  ch = 256
+  lim = math.sqrt(6.0 / (9 * (cx + ch) + 9 * 4 * ch))
+  return dict(kernel=rng.uniform(-lim, lim, size=(3, 3, cx + ch, 4 * ch)).astype(np.float32),
+              biases=(rng.standard_normal(4 * ch) * 0.1).astype(np.float32),
+              x=(rng.standard_normal((ns, h, w, cx), dtype=np.float32) * np.float32(x_scale)),
+              h=np.tanh(rng.standard_normal((ns, h, w, ch), dtype=np.float32)),
+              c=rng.standard_normal((ns, h, w, ch), dtype=np.float32))
+
+
 def checksum(*arrays):
   return float(sum(float(np.sum(np.asarray(a, dtype=np.float64))) for a in arrays))
 
